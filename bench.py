@@ -2,7 +2,7 @@
 """bench.py -- the vAttention hot path on B200, BASELINE.json's metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|fa_vattn]
-                    [--workload decode32k|tp70b] [--ctx C]
+                    [--workload decode32k|tp70b] [--ctx C] [--dump-outputs DIR]
 
 Workload "decode32k" (default; BASELINE.json configs[1]): Llama-3-8B attention shapes (Hq 32,
 Hkv 8, D 128, 32 layers, hidden 4096), batch 64, 32K context, K/V in vAttention virtual tensors
@@ -307,15 +307,15 @@ def run_ours(args):
     # (the wrapper's per-step slice [:, :max_cache_len], vattention_flashattention_wrapper.py:197, with
     # the maximum taken over the whole run)
     static_len = min(max_ctx, max(seq_lens) + total_steps + 8)
+    step_out = [None] * LAYERS                   # the latest step's layer-call outputs (--dump-outputs)
 
     def layers_body(full_views: bool, max_len: int = 0):
-        out = None
         for layer in range(LAYERS):
             kc, vc = k_layers[layer % n_res], v_layers[layer % n_res]
             kc, vc = (kc[:, :static_len], vc[:, :static_len]) if full_views else (kc[:, :max_len], vc[:, :max_len])
-            out = tp_attn.forward(q[layer], kc, vc, kn[layer], vn[layer], cache_seqlens=cs,
-                                  cache_batch_idx=batch_idx, softmax_scale=scale, causal=True)
-        sink.add_(out.flatten()[0].float())
+            step_out[layer] = tp_attn.forward(q[layer], kc, vc, kn[layer], vn[layer], cache_seqlens=cs,
+                                              cache_batch_idx=batch_idx, softmax_scale=scale, causal=True)
+        sink.add_(step_out[-1].flatten()[0].float())
         cs.add_(1)
 
     def eager_step(lens_now):
@@ -370,6 +370,16 @@ def run_ours(args):
     e1.record()
     barrier()
     clocks = sampler.stop() if sampler else None
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed back: every layer-call's block output (the fused and peer
+        # collectives return one internal buffer, valid until the next call: then only the last
+        # layer's survives) and the K/V rows it appended to the resident layers' caches
+        outs = step_out if len({t.data_ptr() for t in step_out}) == LAYERS else step_out[-1:]
+        pos, slots = (cs - 1).long(), batch_idx.long()
+        dumped = {"block_out": torch.stack(outs).cpu(),
+                  "k_appended": torch.stack([t[slots, pos] for t in k_layers]).cpu(),
+                  "v_appended": torch.stack([t[slots, pos] for t in v_layers]).cpu()}
     ms = e0.elapsed_time(e1)
     step_ms = [round(a.elapsed_time(b), 3) for a, b in zip([e0] + marks[:-1], marks)]
     st1 = va.get_step_stats()                     # totals since init_kvcache; the difference is the timed region
@@ -537,9 +547,26 @@ def run_ours(args):
         }
         line.update(extras)
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor as <out_dir>/<name>.npy in float32, so that two builds run with the same
+    arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    total = sum(t.numel() * 4 for t in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().numpy())
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum of ONE launch of decode_tc_kernel on the decode32k
@@ -872,8 +899,8 @@ def run_reference(args):
 # --------------------------------------------------------------------------- fa_vattn ---
 
 def run_fa_vattn(args):
-    """The reference's own GPU path on this box: ITS vattention extension (compiled unmodified from
-    /root/reference/vattention/vattention.cu into oracle/_ref by oracle/Makefile) allocates the virtual
+    """The reference's own GPU path on this box: ITS vattention extension (compiled unmodified from the
+    original project's vattention/vattention.cu into oracle/_ref by oracle/Makefile) allocates the virtual
     tensors and maps the pages; flash_attn.flash_attn_with_kvcache (the library its wrapper dispatches
     to) attends over them.  A comparison arm; nothing of the product is on this path."""
     import glob
@@ -959,7 +986,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the prefill / pod / fa_vattn legs (N = 1)")
     ap.add_argument("--cpu-sample-seqs", type=int, default=2)
     ap.add_argument("--cpu-budget-s", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (float32): "
+                         "block_out [layer-calls, batch, hidden], k_appended / v_appended [resident layers, "
+                         "batch, kv heads, head dim]")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

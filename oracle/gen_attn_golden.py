@@ -3,7 +3,8 @@ un-vendored dependency the reference dispatches to; installed 2.8.3, reference p
 2.5.9.post1) on small seeded inputs.  Runs on the GPU box:
     python oracle/gen_attn_golden.py [outdir]      (default gpurun_out/golden)
 Each file stores the inputs (so the fixture does not depend on RNG reproducibility), the
-library's output and the cache contents after the append.  TEST INFRASTRUCTURE ONLY.
+library's output and the rows its append wrote into the caches (`with_appended` rebuilds the caches
+after the call; the rest of them is unchanged, which is checked here).  TEST INFRASTRUCTURE ONLY.
 """
 import os
 import sys
@@ -27,6 +28,29 @@ CASES = [
 ]
 ROPE = {"rope_decode_neox_bf16": (False, 128), "rope_decode_gptj_fp16": (True, 128),
         "rope_append4_causal_partial_fp16": (False, 64), "rope_append4_noncausal_bf16": (True, 32)}
+
+
+def with_appended(cache, rows, lens, idx):
+    """A copy of `cache` [slots, Sk, Hkv, D] with rows[b] written at rows [lens[b], lens[b] + n) of
+    batch row b's slot (idx[b], or b without an index); `rows` [B, n, Hkv, D] or None."""
+    out = cache.clone()
+    if rows is not None:
+        slots = range(rows.shape[0]) if idx is None else idx.tolist()
+        for b, (s, n) in enumerate(zip(slots, lens.tolist())):
+            out[s, n:n + rows.shape[1]] = rows[b]
+    return out
+
+
+def appended_rows(before, after, lens, idx, n_new):
+    """The rows a call appended to a cache (None without an append); raises if it changed anything
+    else."""
+    rows = None
+    if n_new:
+        slots = range(len(lens)) if idx is None else idx.tolist()
+        rows = torch.stack([after[s, n:n + n_new] for s, n in zip(slots, lens.tolist())])
+    if not torch.equal(with_appended(before, rows, lens, idx), after):
+        raise RuntimeError("the call changed cache rows outside the appended ones")
+    return rows
 
 
 def main(outdir):
@@ -66,7 +90,8 @@ def main(outdir):
                     "q": q, "k_cache": kc, "v_cache": vc, "k": kn, "v": vn, "cache_seqlens": lens,
                     "cache_batch_idx": idx, "causal": causal, "out": out.cpu(),
                     "rotary_cos": cos, "rotary_sin": sin, "rotary_interleaved": interleaved,
-                    "k_cache_after": kc_d.cpu(), "v_cache_after": vc_d.cpu()},
+                    "k_cache_appended": appended_rows(kc, kc_d.cpu(), lens, idx, n_new),
+                    "v_cache_appended": appended_rows(vc, vc_d.cpu(), lens, idx, n_new)},
                    os.path.join(outdir, f"attn_{name}.pt"))
         print(name, tuple(out.shape))
 

@@ -1,5 +1,5 @@
 """Replay an allocator API trace on the REFERENCE extension (oracle/_ref/vattention_ref*.so,
-built unmodified from /root/reference/vattention/vattention.cu by oracle/Makefile) and dump
+built unmodified from the original project's vattention/vattention.cu by oracle/Makefile) and dump
 its state after every call as JSON.
 
 TEST INFRASTRUCTURE ONLY.  Runs on the GPU box (the module needs libcuda).  State that the
@@ -29,7 +29,7 @@ def load_ref():
     here = os.path.dirname(os.path.abspath(__file__))
     cands = glob.glob(os.path.join(here, "_ref", "vattention_ref*.so"))
     if not cands:
-        raise SystemExit("oracle/_ref/vattention_ref*.so not built (run `make -C oracle`)")
+        raise SystemExit("oracle/_ref/vattention_ref*.so not built (run `make -C oracle REF=<checkout>/vattention`)")
     import torch  # noqa: F401  (libtorch must be loaded first)
     spec = importlib.util.spec_from_file_location("vattention_ref", cands[0])
     mod = importlib.util.module_from_spec(spec)
